@@ -414,9 +414,10 @@ def gpu_run(args):
     table = DeviceTable(lib, space, dev, my_days, rows_per_batch, WL.get("city_dist", "uniform"), mirror_host=not args.no_e2e)
     zone_map_ms = table.zone_map_ms
 
-    def run_workload(name, steps, warmup, zone_maps, table, with_kernel=True, with_e2e=False, verify=True, rows_scale=1):
+    def run_workload(name, steps, warmup, zone_maps, table, with_kernel=True, with_e2e=False, verify=True, rows_scale=1,
+                     dump_dir=None):
         """Times one workload on `table`; returns the sub-result dict (device-resident value, kernel-alone roofline,
-        optional e2e, verification)."""
+        optional e2e, verification).  dump_dir: where to write the result of the last timed step (dump_outputs)."""
         wl = WORKLOADS[name]
         q = wl["query"]()
         nb = wl["batches"]
@@ -476,6 +477,12 @@ def gpu_run(args):
         if name == args.workload and args.profile_range:
             torch.cuda.synchronize()
             torch.cuda.profiler.stop()
+        if dump_dir and rank == 0:
+            if q.is_hll:
+                dump_outputs(dump_dir, last)
+            else:
+                g, bufs = last
+                dump_outputs(dump_dir, QueryResult(q, bufs.dims.get(np.uint8), bufs.capacity, bufs.measures.get(np.uint8), g))
         out = {"value": rows_all / (ms / 1e3), "unit": "rows/s", "ms_per_step": ms, "p50_query_ms": float(np.median(per)),
                "step_ms": [round(x, 4) for x in per],
                "steps": steps, "gpu_launches": int(launches), "zone_maps": bool(zone_maps)}
@@ -606,7 +613,8 @@ def gpu_run(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    main = run_workload(args.workload, args.steps, args.warmup, not args.no_zone_maps, table, with_e2e=not args.no_e2e)
+    main = run_workload(args.workload, args.steps, args.warmup, not args.no_zone_maps, table, with_e2e=not args.no_e2e,
+                        dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     subs = {}
@@ -680,6 +688,50 @@ def gpu_run(args):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res):
+    """Writes the groups of a QueryResult / HLLResult as DIR/<name>.npy, one row per group, ordered by the packed
+    dimension row (the order a hash table hands groups out in is not part of the result), so that two builds can be
+    compared array for array:
+        dim<i>        float64, the i-th dimension's value (NaN for NULL)
+        measures      float64 (SUM / COUNT / MIN / MAX / AVG), counts float64 for AVG
+        hll_counts    float64, non-zero registers per group;  hll_registers float32 [groups, 16384], rho + 1 per register
+    Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of the groups is written and group_index names its rows."""
+    from aresdb_b200.query import HLLResult
+    hll = isinstance(res, HLLResult)
+    qr = res.dims if hll else res
+    rows = qr.packed_rows()
+    order = np.lexsort(rows.T[::-1]) if rows.shape[1] else np.arange(qr.groups)
+    arrays = {}
+    for i, col in enumerate(qr.decoded_dims()):
+        arrays[f"dim{i}"] = np.array([np.nan if v is None else float(v) for v in col], np.float64)[order]
+    if hll:
+        dense = res.dense_registers()
+        arrays["hll_counts"] = res.counts.astype(np.float64)[order]
+        arrays["hll_registers"] = np.stack([dense[qr.rows[g]] for g in order]).astype(np.float32) if qr.groups \
+            else np.zeros((0, 1 << 14), np.float32)
+    else:
+        arrays["measures"] = qr.measures.astype(np.float64)[order]
+        if qr.counts is not None:
+            arrays["counts"] = qr.counts.astype(np.float64)[order]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = int(qr.groups * DUMP_LIMIT_BYTES // (total + 8 * qr.groups))     # 8 bytes more per row: group_index
+        idx = np.sort(np.random.default_rng(0).choice(qr.groups, size=keep, replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["group_index"] = idx.astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for f in out.glob("*.npy"):      # what an earlier dump left (another workload's dims, a sample's group_index)
+        if f.stem in ("measures", "counts", "hll_counts", "hll_registers", "group_index") or \
+                (f.stem.startswith("dim") and f.stem[3:].isdigit()):
+            f.unlink()
+    for k, v in arrays.items():
+        np.save(out / f"{k}.npy", v)
+
+
 PEAK, PEAK_SRC = 6650.0, "fallback 6650 GB/s"
 
 
@@ -729,7 +781,11 @@ def main():
     ap.add_argument("--no-sub", action="store_true", help="N = 1: skip the sub-results of the other BASELINE configs")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling leg (1e9 rows per GPU)")
     ap.add_argument("--no-zipf", action="store_true", help="skip the Zipf-city sub-result (a second 11.5 GB table)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="B200 path: write the result of the last timed step of --workload as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     select_workload(args.workload)
     _load_peak()
     if args.impl == "reference":

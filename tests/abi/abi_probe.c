@@ -1,9 +1,8 @@
 /* abi_probe.c — prints size / field offsets of every by-value struct and the values of the ABI enums of the cgo boundary.
- * Compiled TWICE by tests/test_abi_vs_reference_headers.py: once against the REFERENCE's own headers
- * (-DUSE_REFERENCE -I/root/reference: query/time_series_aggregate.h + cgoutils/memory.h) and once against
- * include/aresdb_b200/*.h; the two outputs must be identical.  The reference build of this file is also LINKED against
- * aresdb_b200/lib/libalgorithm.so + libmem.so and calls entry points through the reference's own prototypes: a
- * translation unit that only ever saw the reference's headers binds to the B200 libraries unchanged. */
+ * Compiled against the REFERENCE's own headers (-DUSE_REFERENCE -I<reference tree>: query/time_series_aggregate.h +
+ * cgoutils/memory.h), its output is tests/golden/abi_layout_reference.txt; tests/test_abi_vs_reference_headers.py
+ * compiles it against include/aresdb_b200/*.h and requires the same output.  It also LINKS this file against
+ * aresdb_b200/lib/libalgorithm.so + libmem.so and calls entry points through the declared prototypes. */
 #include <stddef.h>
 #include <stdio.h>
 #ifdef USE_REFERENCE

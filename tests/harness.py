@@ -44,7 +44,7 @@ def get_backend(name: str) -> Backend:
     if name == "ref":
         alg, mem = REF_DIR / "libalgorithm.so", REF_DIR / "libmem_ref.so"
         if not alg.exists():
-            pytest.skip("oracle/_ref not built (needs /root/reference; run oracle/build_ref.sh)")
+            pytest.skip("oracle/_ref not built (ARESDB_REFERENCE=<reference tree> bash oracle/build_ref.sh)")
         return Backend("ref", cabi.Library(alg, mem, has_plan_api=False, name="ref"), HostSpace())
     if name == "oracle":
         if not ORACLE_LIB.exists():

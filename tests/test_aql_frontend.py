@@ -10,6 +10,8 @@ import numpy as np
 import pytest
 
 import harness as H
+import reference_golden as R
+from reference_golden import reference_results  # noqa: F401  (autouse fixture)
 from aresdb_b200 import aql, cabi as A, columns, expr as E
 from aresdb_b200.executor import Batch, FusedBatchExecutor, LegacyBatchExecutor
 
@@ -269,10 +271,12 @@ def test_one_switch_in_range_builds_the_references_expression_and_evaluates_to_i
     exp = {}
     for b in (local[keep] // 3600 * 3600).tolist():
         exp[b] = exp.get(b, 0) + 1
-    for backend in ("ref", "oracle"):
-        res = T.run_legacy(H.get_backend(backend), agg, [hb])
-        got = dict(zip(np.array(res.decoded_dims()[0], np.int64).tolist(), res.measures.tolist()))
-        assert got == exp and len(got) > 20, backend
+    def hours(be):
+        res = T.run_legacy(be, agg, [hb])
+        return dict(zip(np.array(res.decoded_dims()[0], np.int64).tolist(), res.measures.tolist()))
+    got = hours(H.get_backend("oracle"))
+    assert got == exp and len(got) > 20
+    R.assert_same(exp, R.expected(hours), "reference HOST build")
     # numeric output back to instants (utils.AdjustOffset): buckets before the switch by the from-offset, later ones by the to-offset
     meta = DimensionMeta(time_bucketizer="hour", time_unit="second", from_offset=-25200, to_offset=-28800, dst_switch=1_509_872_400)
     assert format_time_dimension(1_509_872_400 - 28800 - 3600, meta) == str(1_509_872_400 - 28800 - 3600 + 25200)
@@ -345,10 +349,11 @@ def test_in_lists_null_tests_and_bitwise_operators_end_to_end():
         for s_, ok in zip(status[keep].tolist(), vs[keep].tolist()):
             k = s_ if ok else None
             exp[k] = exp.get(k, 0) + 1
-        for backend in ("ref", "oracle"):
-            res = T.run_legacy(H.get_backend(backend), agg, [hb])
-            got = dict(zip(res.decoded_dims()[0], res.measures.tolist()))
-            assert got == exp, (text, backend)
+        def groups(be):
+            res = T.run_legacy(be, agg, [hb])
+            return dict(zip(res.decoded_dims()[0], res.measures.tolist()))
+        assert groups(H.get_backend("oracle")) == exp, text
+        R.assert_same(exp, R.expected(groups), f"{text}: reference HOST build")
     for bad in ("fare + 1 in (2)", "city_id not 3", "fare is 3", "city_id in 1"):
         with pytest.raises(aql.AQLError):
             aql.parse_expression(bad, table)

@@ -10,6 +10,7 @@ import pytest
 import harness as H
 import test_pipeline_parity as T
 from aresdb_b200 import archive as AR
+from reference_golden import reference_results  # noqa: F401  (autouse fixture)
 from aresdb_b200 import cabi as A
 from aresdb_b200 import expr as E, synth
 from aresdb_b200.executor import LegacyBatchExecutor
@@ -194,21 +195,27 @@ def test_archive_scan_evaluates_the_time_filter_on_the_first_and_last_day_only()
     assert archive.archive_batch_ids((frm, None), synth.BASE_TS + 2 * 86400 + 5).stop == day0 + 3
     # (an archive batch's time column is never NULL and lies inside its day: that is what makes the rule exact)
     hbs = {day0 + d: synth.generate_batch(d, 3000 + 500 * d, num_cities=6, null_rate=0.0) for d in range(6)}
-    for backend in ("ref", "oracle"):
-        be = H.get_backend(backend)
-        results = []
+    def scans(be):
+        results = {}
         for rule in (True, False):
             ex = LegacyBatchExecutor(be.lib, be.space, q)
             keep = {day: T.upload(be, hb) for day, hb in hbs.items()}
             if rule:
-                done = archive.scan_archive_batches(ex, keep, q.time_range, 0)
-                assert done == [(day0 + 1, True), (day0 + 2, False), (day0 + 3, False), (day0 + 4, True)]
+                results["done"] = [list(d) for d in archive.scan_archive_batches(ex, keep, q.time_range, 0)]
             else:
                 for day in archive.archive_batch_ids(q.time_range, 0):
                     ex.process_batch(keep[day])
-            results.append(ex.result())
-        assert results[0].groups > 60
-        T.assert_same_result(results[0], results[1], ctx=backend)
+            results["rule" if rule else "every batch"] = ex.result()
+        return results
+    import reference_golden as R
+    want_done = [[day0 + 1, True], [day0 + 2, False], [day0 + 3, False], [day0 + 4, True]]
+    got = scans(H.get_backend("oracle"))
+    assert got["done"] == want_done and got["rule"].groups > 60
+    T.assert_same_result(got["rule"], got["every batch"], ctx="oracle")
+    exp = R.expected(scans)                                # the reference's HOST build
+    assert exp["done"] == want_done and exp["rule"]["groups"] > 60
+    R.assert_same_result(got["every batch"], exp["every batch"], ctx="reference, every batch")
+    R.assert_same_result(got["every batch"], exp["rule"], ctx="reference, first / last day rule")
 
 
 @pytest.mark.gpu
@@ -273,21 +280,24 @@ def test_shard_scan_live_batches_with_the_cutoff_filter_then_archive_days():
     ranges = {"both": (synth.BASE_TS + 86400 + 1800, synth.BASE_TS + 5 * 86400 - 1800),
               "archive only": (synth.BASE_TS + 3600, synth.BASE_TS + 2 * 86400),
               "live only": (cutoff + 7200, cutoff + 2 * 86400)}
-    for backend in ("ref", "oracle"):
-        be = H.get_backend(backend)
-        for name, (frm, to) in ranges.items():
-            text = {"table": "trips", "measures": [{"sqlExpression": "count(*)"}],
-                    "timeFilter": {"column": "request_at", "from": str(frm), "to": str(to - 1)},
-                    "dimensions": [{"sqlExpression": "request_at", "timeBucketizer": "hour"}]}
-            q = aql.compile_query(text, table, synth.BASE_TS + 30 * 86400)
-            frm, to = q.time_range
+    import reference_golden as R
+    for name, (frm, to) in ranges.items():
+        text = {"table": "trips", "measures": [{"sqlExpression": "count(*)"}],
+                "timeFilter": {"column": "request_at", "from": str(frm), "to": str(to - 1)},
+                "dimensions": [{"sqlExpression": "request_at", "timeBucketizer": "hour"}]}
+        q = aql.compile_query(text, table, synth.BASE_TS + 30 * 86400)
+        frm, to = q.time_range
+
+        def scan(be):
             ex = LegacyBatchExecutor(be.lib, be.space, q)
-            done = archive.scan_shard(ex, [T.upload(be, hb) for hb in live], {d: T.upload(be, hb) for d, hb in arch.items()}, cutoff,
-                                      q.time_range, 0)
-            assert (done["live"] > 0) == (name != "archive only") and (len(done["archive"]) > 0) == (name != "live only")
+            done = archive.scan_shard(ex, [T.upload(be, hb) for hb in live], {d: T.upload(be, hb) for d, hb in arch.items()},
+                                      cutoff, q.time_range, 0)
             res = ex.result()
-            got = dict(zip(np.array(res.decoded_dims()[0], np.int64).tolist(), res.measures.tolist()))
-            assert got == expected(frm, to) and len(got) > 10, (backend, name)
+            return {"live": done["live"] > 0, "archive": len(done["archive"]) > 0,
+                    "hours": dict(zip(np.array(res.decoded_dims()[0], np.int64).tolist(), res.measures.tolist()))}
+        want = {"live": name != "archive only", "archive": name != "live only", "hours": expected(frm, to)}
+        assert scan(H.get_backend("oracle")) == want and len(want["hours"]) > 10, name
+        R.assert_same(want, R.expected(scan), f"{name}: reference HOST build")
     # the cutoff filter is one more filter instruction, ahead of the time filters
     assert len(q.plan_instructions(cutoff=cutoff)) == len(q.plan_instructions()) + 1
 

@@ -9,6 +9,8 @@ import numpy as np
 import pytest
 
 import harness as H
+import reference_golden as R
+from reference_golden import reference_results  # noqa: F401  (autouse fixture)
 import test_pipeline_parity as T
 from aresdb_b200 import cabi as A, columns, expr as E, joins as J, synth
 from aresdb_b200.query import AggQuery, Join, Measure
@@ -127,14 +129,13 @@ def host_batches():
 
 @pytest.mark.parametrize("name", ["by_region", "local_hour", "sum_surge", "unmatched"])
 def test_join_sequence_oracle_vs_reference(name, host_batches):
-    ref, orc = H.get_backend("ref"), H.get_backend("oracle")
-    res = []
-    for be in (ref, orc):
+    def run(be):
         table, _ = _dimension_table(be)
         tzb, tzn = _tz_table(be)
-        res.append(T.run_legacy(be, join_queries(table, tzb.ptr, tzn)[name], host_batches))
-    assert res[0].groups > 0
-    T.assert_same_result(res[1], res[0], ctx=name)
+        return T.run_legacy(be, join_queries(table, tzb.ptr, tzn)[name], host_batches)
+    exp = R.expected(run)
+    assert exp["groups"] > 0
+    R.assert_same_result(run(H.get_backend("oracle")), exp, ctx=name)
 
 
 @pytest.mark.gpu

@@ -10,6 +10,8 @@ import numpy as np
 import pytest
 
 import harness as H
+import reference_golden as R
+from reference_golden import reference_results  # noqa: F401  (autouse fixture)
 from aresdb_b200 import cabi as A
 from aresdb_b200 import columns, expr as E, synth
 from aresdb_b200.executor import Batch, FusedBatchExecutor, LegacyBatchExecutor
@@ -94,12 +96,12 @@ def host_batches():
 @pytest.mark.parametrize("name", list(queries()))
 def test_legacy_sequence_oracle_vs_reference(name, host_batches):
     """CPU: pins the Python driver + the C restatement against the reference's HOST build."""
-    ref, orc = H.get_backend("ref"), H.get_backend("oracle")
+    orc = H.get_backend("oracle")
     q = queries()[name]
-    exp = run_legacy(ref, q, host_batches)
+    exp = R.expected(lambda ref: run_legacy(ref, q, host_batches))
     got = run_legacy(orc, q, host_batches)
-    assert exp.groups > 0
-    assert_same_result(got, exp, ordered=q.reduce_mode == A.ARES_REDUCE_SORT, ctx=name)
+    assert exp["groups"] > 0
+    R.assert_same_result(got, exp, ordered=q.reduce_mode == A.ARES_REDUCE_SORT, ctx=name)
 
 
 @pytest.mark.gpu
@@ -197,16 +199,25 @@ def test_zone_map_null_dimensions_and_replicas():
 def test_negative_zero_sums_oracle_vs_reference():
     """CPU: a group whose fares are all -0.0 sums to -0.0 through Sort + Reduce and to +0.0 through HashReduce (its map
     folds into a slot that starts at +0.0) — pinned on the reference's HOST build, the GPU test below relies on it."""
-    ref, orc = H.get_backend("ref"), H.get_backend("oracle")
+    orc = H.get_backend("oracle")
     hbs = [synth.generate_batch(0, 4000, num_cities=40, null_rate=0.05)]
     hbs[0].values[synth.COL_FARE][::3] = np.float32(-0.0)
     dims = [CITY, E.floor(TS, E.Lit(60))]
+
+    def zero_signs(r):
+        return np.signbit(r.measures[r.measures == 0])
+
+    def with_signs(r):
+        s = zero_signs(r)
+        return {"result": r, "zeros": int(s.size), "negative_zeros": int(s.sum())}
+
     for mode in (A.ARES_REDUCE_SORT, A.ARES_REDUCE_HASH):
         q = AggQuery([], dims, Measure("sum", FARE), reduce_mode=mode)
-        exp, got = run_legacy(ref, q, hbs), run_legacy(orc, q, hbs)
-        assert_same_result(got, exp, ordered=mode == A.ARES_REDUCE_SORT, ctx=f"-0.0 sums, mode {mode}")
-        signs = np.signbit(exp.measures[exp.measures == 0])
-        assert signs.size > 0 and (signs.any() if mode == A.ARES_REDUCE_SORT else not signs.any())
+        exp, got = R.expected(lambda ref: with_signs(run_legacy(ref, q, hbs))), run_legacy(orc, q, hbs)
+        R.assert_same_result(got, exp["result"], ordered=mode == A.ARES_REDUCE_SORT, ctx=f"-0.0 sums, mode {mode}")
+        assert exp["zeros"] > 0 and (exp["negative_zeros"] > 0 if mode == A.ARES_REDUCE_SORT else exp["negative_zeros"] == 0)
+        signs = zero_signs(got)
+        assert signs.size == exp["zeros"] and signs.sum() == exp["negative_zeros"]
 
 
 @pytest.mark.gpu
@@ -378,13 +389,16 @@ def test_fused_plan_on_archive_style_batches(name, runs):
 
 @pytest.mark.parametrize("name", ["cfg2", "cfg3_count"])
 def test_archive_style_batches_oracle_vs_reference(name):
-    ref, orc = H.get_backend("ref"), H.get_backend("oracle")
+    orc = H.get_backend("oracle")
     q = queries()[name]
-    a, b = LegacyBatchExecutor(ref.lib, ref.space, q), LegacyBatchExecutor(orc.lib, orc.space, q)
-    a.process_batch(_archive_batch(ref, 1))
-    b.process_batch(_archive_batch(orc, 1))
-    assert a.result().groups > 0
-    assert_same_result(b.result(), a.result(), ctx=f"archive/{name}")
+
+    def run(be):
+        ex = LegacyBatchExecutor(be.lib, be.space, q)
+        ex.process_batch(_archive_batch(be, 1))
+        return ex.result()
+    exp = R.expected(run)
+    assert exp["groups"] > 0
+    R.assert_same_result(run(orc), exp, ctx=f"archive/{name}")
 
 
 # ---- AVG: (float average, count) pairs combined with the reference's rolling average -------------------
@@ -409,11 +423,12 @@ def assert_same_avg(got, exp, ctx="", exact=False):
 
 @pytest.mark.parametrize("name", list(avg_queries()))
 def test_avg_sequence_oracle_vs_reference(name, host_batches):
-    ref, orc = H.get_backend("ref"), H.get_backend("oracle")
+    orc = H.get_backend("oracle")
     q = avg_queries()[name]
-    exp, got = run_legacy(ref, q, host_batches), run_legacy(orc, q, host_batches)
-    assert exp.groups > 0 and exp.counts.sum() > 0
-    assert_same_avg(got, exp, name, exact=True)
+    exp, got = R.expected(lambda ref: run_legacy(ref, q, host_batches)), run_legacy(orc, q, host_batches)
+    assert exp["groups"] > 0 and got.counts.sum() > 0
+    R.assert_same_result(got, exp, ctx=name)      # rows, counts and averages bit for bit
+    exp = got
     # and the averages are what they should be
     hb = host_batches
     if name == "avg_fare_by_city":
@@ -481,14 +496,17 @@ def mixed_queries():
 
 @pytest.mark.parametrize("name", list(mixed_queries()))
 def test_mixed_column_modes_oracle_vs_reference(name):
-    ref, orc = H.get_backend("ref"), H.get_backend("oracle")
+    orc = H.get_backend("oracle")
     q = mixed_queries()[name]
-    a, b = LegacyBatchExecutor(ref.lib, ref.space, q), LegacyBatchExecutor(orc.lib, orc.space, q)
-    for seed in (1, 2):
-        a.process_batch(_mixed_batch(ref, seed))
-        b.process_batch(_mixed_batch(orc, seed))
-    assert a.result().groups > 1
-    assert_same_result(b.result(), a.result(), ctx=name)
+
+    def run(be):
+        ex = LegacyBatchExecutor(be.lib, be.space, q)
+        for seed in (1, 2):
+            ex.process_batch(_mixed_batch(be, seed))
+        return ex.result()
+    exp = R.expected(run)
+    assert exp["groups"] > 1
+    R.assert_same_result(run(orc), exp, ctx=name)
 
 
 @pytest.mark.gpu
